@@ -150,15 +150,15 @@ def small_complete_cpu(cores):
 
 
 def try_tlc(seconds):
-    """BASELINE.md: if a JVM and tla2tools.jar ever appear on the box ($TLA2TOOLS_JAR) together with the spec ($VSR_TLA, or the
-    reference checkout), run the REAL reference — TLC — on the same config for a bounded time and return its rate.  In this
+    """BASELINE.md: if a JVM and tla2tools.jar ever appear on the box ($TLA2TOOLS_JAR) together with the spec ($VSR_TLA),
+    run the REAL reference — TLC — on the same config for a bounded time and return its rate.  In this
     image there is no java, so this returns None and the CPU restatement stands in."""
     import re
     import shutil
     import tempfile
     jar, java = os.environ.get("TLA2TOOLS_JAR"), shutil.which("java")
-    tla = os.environ.get("VSR_TLA", "/root/reference/vsr-revisited/paper/VSR.tla")
-    if not (jar and java and os.path.exists(jar) and os.path.exists(tla)):
+    tla = os.environ.get("VSR_TLA")
+    if not (jar and java and tla and os.path.exists(jar) and os.path.exists(tla)):
         return None
     import _pkg
     pkg = _pkg.load()
@@ -261,6 +261,42 @@ def golden_depths(pkg, mc, eng, torch, tdist, world, dev, rank):
     return [int(x) for x in t.cpu().tolist()]
 
 
+def sampled_state_depths(mc, eng, torch, tdist, world, dev, rank, walks=64, steps=64, seed=0):
+    """BFS depth at which the seen-set holds each state of a fixed sample of the reachable set (0 = absent): the states of
+    `walks` seeded random walks of `steps` steps from Init through the host's Next, successors taken in byte order so that
+    the sample does not depend on the order a build lists them in"""
+    import random
+    rng = random.Random(seed)
+    sample = []
+    for _ in range(walks):
+        s = mc.init_state()
+        for _ in range(steps):
+            sample.append(s)
+            succ = sorted(t for t, _, _ in mc.successors(s))
+            if not succ:
+                break
+            s = rng.choice(succ)
+    levels = []
+    for s in sample:
+        lvl, owner = eng.lookup(s)
+        levels.append(lvl if owner == rank else 0)
+    t = torch.tensor(levels, dtype=torch.int64, device=dev)
+    if world > 1:
+        tdist.all_reduce(t, op=tdist.ReduceOp.MAX)
+    return t.cpu().numpy()
+
+
+def dump_outputs(path, res, depths):
+    """what the timed path returned in its last step, as float64 .npy files (exact: every count is below 2^53)"""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    totals = [res.rc, res.generated, res.distinct, res.queue, res.depth, res.complete, res.violation_level, res.h2_ties, res.fp_collisions]
+    out = {"totals": totals,  # rc, generated, distinct, queue, depth, complete, violation_level, h2_ties, fp_collisions
+           "level_sizes": res.level_sizes, "level_generated": res.level_generated, "sampled_state_depths": depths}
+    for name, a in out.items():
+        np.save(os.path.join(path, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def cfg3_first_violation(pkg, vdist, torch, tdist, group, rank, world, local, dev, barrier):
     """BASELINE configs[2]/[4]: the README constants (the config the reference says needs 500 GB of disk and days under TLC)
     sharded over the job's GPUs, to the first AcknowledgedWriteNotLost violation; the published trace's states must be in
@@ -314,10 +350,15 @@ def main():
                     help="N = 1: run that block too: 3.17e9 states on ONE GPU with the frontier spilling into 109 GB of pinned host memory "
                          "(off by default: a box that is a slice of a machine may not have that much)")
     ap.add_argument("--no-e2e", action="store_true", help="profiling runs: skip the end-to-end legs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (float64): totals, level_sizes, "
+                         "level_generated, and the seen-set's depth of a fixed seeded sample of states")
     ap.add_argument("--exchange", default="p2p", choices=["p2p", "staged"],
                     help="N > 1: p2p = the kernel stores remote successors into the owner's inbox over NVLink, C++ level loop (default); "
                          "staged = the baseline it replaces: local staging buffer + NCCL send/recv per step, Python level loop")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -394,6 +435,10 @@ def main():
     wall = float(t[0])
     clocks = sampler.stop() if rank == 0 else None
     st = eng.stats()
+    if args.dump_outputs:
+        depths = sampled_state_depths(mc, eng, torch, tdist, world, dev, rank)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, res, depths)
 
     ok = (res.distinct == EXPECT["distinct"] and res.generated == EXPECT["generated"] and res.depth == EXPECT["depth"] and
           res.violation_level == EXPECT["violation_level"] and res.complete)

@@ -7,10 +7,11 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 
-REFERENCE = "/root/reference"
-REF_TLA = os.path.join(REFERENCE, "vsr-revisited/paper/VSR.tla")
-REF_CFG = os.path.join(REFERENCE, "vsr-revisited/paper/VSR.cfg")
-REF_TRACE = os.path.join(REFERENCE, "state_transfer_violation_trace.txt")
+GOLDEN = os.path.join(ROOT, "tests", "golden")
+# data files of the upstream project (Vanlightly/vsr-tlaplus), stored unchanged: the shipped model configuration and the
+# published 24-state counterexample
+REF_CFG = os.path.join(GOLDEN, "VSR.cfg")
+REF_TRACE = os.path.join(GOLDEN, "state_transfer_violation_trace.txt")
 
 
 def pytest_configure(config):
@@ -26,11 +27,3 @@ def pkg():
         import __graft_entry__
         __graft_entry__.build()
     return _pkg.load()
-
-
-@pytest.fixture(scope="session")
-def have_reference():
-    return os.path.exists(REF_TLA)
-
-
-needs_reference = pytest.mark.skipif(not os.path.exists(REF_TLA), reason="/root/reference is not mounted here")

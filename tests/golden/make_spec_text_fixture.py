@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Generates tests/golden/spec_text_results.json: what oracle/tla_eval.py derives from the TEXT of the reference's
-vsr-revisited/paper/VSR.tla (read from /root/reference — this script only runs where the reference is mounted).
+vsr-revisited/paper/VSR.tla (read from the vsr-tlaplus checkout that VSR_TLAPLUS_DIR names).
 
   state_spaces   level sizes / successors generated per level / totals of breadth-first searches run by the text
                  evaluator (SYMMETRY off, VIEW on), complete for the small configurations, depth-bounded for bigger ones
@@ -10,10 +10,10 @@ vsr-revisited/paper/VSR.tla (read from /root/reference — this script only runs
                  behaviour of the text (action names of profiles/cfg2_counterexample)
 
 tests/test_spec_text.py::test_oracle_equals_the_committed_spec_text_results checks the oracle against `state_spaces`
-on every machine (the GPU box has no /root/reference).
+on every machine.
 
-    python tests/golden/make_spec_text_fixture.py                          # everything (about 20 minutes)
-    python tests/golden/make_spec_text_fixture.py --add-space R V L DEPTH  # one more state space (DEPTH 0 = complete)
+    VSR_TLAPLUS_DIR=<checkout> python tests/golden/make_spec_text_fixture.py                          # everything (about 20 minutes)
+    VSR_TLAPLUS_DIR=<checkout> python tests/golden/make_spec_text_fixture.py --add-space R V L DEPTH  # one more state space (DEPTH 0 = complete)
 """
 import base64
 import json
@@ -44,6 +44,7 @@ def space_row(R, V, L, depth):
 
 
 def main():
+    assert S.LIVE, "set VSR_TLAPLUS_DIR to a vsr-tlaplus checkout"
     pkg = _pkg.load()
     if len(sys.argv) == 6 and sys.argv[1] == "--add-space":  # one more state space into the existing file (long runs)
         R, V, L, depth = map(int, sys.argv[2:6])

@@ -1,10 +1,10 @@
 #!/usr/bin/env python
 """Generates tests/golden/state_transfer_trace.json from the reference's only golden vector,
-/root/reference/state_transfer_violation_trace.txt (24 states, TLC `dumpTrace tlc` text).
+state_transfer_violation_trace.txt (24 states, TLC `dumpTrace tlc` text; stored unchanged beside this script).
 
 The reference file is parsed with the oracle's TLC-value parser; each state is stored as the raw bytes
 of a VsrFlatState (include/vsr_flat.h; zlib + base64, the struct is mostly zeros) next to its action
-name.  The fixture travels to the GPU box, where /root/reference does not exist.
+name.
 
     python tests/golden/make_trace_fixture.py
 """
@@ -23,7 +23,7 @@ sys.path.insert(0, os.path.join(ROOT, "tests"))
 import _pkg  # noqa: E402
 import orc  # noqa: E402
 
-SRC = "/root/reference/state_transfer_violation_trace.txt"
+SRC = os.path.join(HERE, "state_transfer_violation_trace.txt")
 
 
 def main():

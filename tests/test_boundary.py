@@ -7,7 +7,7 @@ import subprocess
 
 import pytest
 
-from conftest import REF_CFG, REF_TLA, ROOT, needs_reference
+from conftest import GOLDEN, REF_CFG, ROOT
 
 HDR = os.path.join(ROOT, "include", "vsr_b200.h")
 
@@ -34,64 +34,103 @@ def test_struct_mirrors_match_c_sizes(pkg, tmp_path):
                      C.sizeof(ck.VsrStats), C.sizeof(ck.VsrLevelInfo)]
 
 
-@needs_reference
-def test_shipped_cfg_and_spec_load_unchanged(pkg):
-    mc = pkg.ModelChecker.from_cfg(REF_CFG, REF_TLA)
+def test_shipped_cfg_loads_unchanged(pkg):
+    mc = pkg.ModelChecker.from_cfg(REF_CFG)
     i = mc.info
     assert (i.replica_count, i.client_count, i.value_count, i.start_view_on_timer_limit, i.restart_empty_limit) == (3, 1, 2, 2, 0)
-    assert (i.symmetry, i.view, i.invariant, i.spec_verified) == (1, 1, 1, 1)
-    assert i.spec_hash == 0x0C8FE64CCA77C791
+    assert (i.symmetry, i.view, i.invariant, i.spec_verified) == (1, 1, 1, 0)  # no .tla given: nothing verified
     assert [bytes(i.value_names[k]).split(b"\0")[0] for k in range(2)] == [b"v1", b"v2"]
     assert i.state_bytes == 48
-    assert mc.action_location(1) == "line 579, col 5 to line 590, col 56 of module VSR"   # TimerSendSVC, VSR.tla:579-590
-    assert mc.action_location(0) == "Unknown location"
 
 
-@needs_reference
-def test_an_edited_spec_is_refused_not_verified(pkg, tmp_path, monkeypatch):
-    """Next and the invariants are hand-lowered, so a .tla whose definitions differ from VSR.tla must not load as "verified"
-    (ADVICE round 1): an edited invariant body keeps the module name, the VARIABLES and the disjunct names."""
-    text = open(REF_TLA).read()
-    edited = text.replace("AcknowledgedWriteNotLost ==", "AcknowledgedWriteNotLost == TRUE \\/", 1)
-    assert edited != text
-    p = tmp_path / "VSR.tla"
-    p.write_text(edited)
+# The 20 VARIABLES of VSR.tla in declaration order and the 19 disjuncts of Next: what the loader checks a .tla against.
+VARIABLES = ["replicas", "rep_status", "rep_log", "rep_view_number", "rep_op_number", "rep_commit_number", "rep_peer_op_number",
+             "rep_client_table", "rep_last_normal_view", "rep_svc_recv", "rep_dvc_recv", "rep_sent_dvc", "rep_sent_sv",
+             "rep_rec_number", "rep_rec_recv", "clients", "messages", "aux_svc", "aux_restart", "aux_client_acked"]
+
+
+def stand_in_spec(pkg, module="VSR"):
+    """A module with VSR.tla's outline (module name, VARIABLES, the action definitions, the disjuncts of Next, the
+    definitions a cfg may name) and bodies of its own: not the spec the checker was lowered from.  Each action body is two
+    lines, `    /\\ <action>_enabled` and `    /\\ UNCHANGED vars` (columns 5 to 21 of the second)."""
+    lines = ["---- MODULE %s ----" % module, "EXTENDS Naturals", "VARIABLES " + ", ".join(VARIABLES), "",
+             "vars == <<" + ", ".join(VARIABLES) + ">>", "", "Init == TRUE", ""]
+    for a in pkg.ACTION_NAMES[1:]:
+        lines += [a + " ==", "    /\\ %s_enabled" % a, "    /\\ UNCHANGED vars", ""]
+    lines += ["Next =="] + ["    \\/ " + a for a in pkg.ACTION_NAMES[1:]] + [""]
+    for d in ("view", "symmValues", "AcknowledgedWriteNotLost", "AcknowledgedWritesExistOnMajority", "NoLogDivergence", "TestInv"):
+        lines.append(d + " == TRUE")
+    return "\n".join(lines + ["===="]) + "\n"
+
+
+def normalised_hash_of_refused(pkg, path):
     with pytest.raises(pkg.VsrError) as ei:
-        pkg.ModelChecker.from_cfg(REF_CFG, str(p))
-    assert ei.value.rc == 150 and "hand" in str(ei.value)
-    # comments, blank lines, trailing blanks and CRLF line ends are not the spec
-    p.write_text("\n".join(("\\* a comment line\n" + ln + "   \r") if i == 200 else ln + "\r" for i, ln in enumerate(text.split("\n"))) + "\n(* block\n comment *)\n")
-    assert pkg.ModelChecker.from_cfg(REF_CFG, str(p)).info.spec_verified == 1
-    # explicit override: loads, loudly, and is NOT reported as verified
-    p.write_text(edited)
+        pkg.ModelChecker.from_cfg(REF_CFG, str(path))
+    assert ei.value.rc == 150 and "hand" in str(ei.value), str(ei.value)
+    return re.search(r"normalised text hash ([0-9a-f]{16})", str(ei.value)).group(1)
+
+
+def test_an_edited_spec_is_refused_and_comments_are_not_the_spec(pkg, tmp_path, monkeypatch):
+    """Next and the invariants are hand-lowered, so a .tla whose text differs from VSR.tla must not load as "verified"
+    even when it keeps the module name, the VARIABLES and the disjunct names; the text is compared after dropping
+    comments, blank lines, trailing blanks and CR, and an edited definition body changes it."""
+    text = stand_in_spec(pkg)
+    p = tmp_path / "VSR.tla"
+    p.write_text(text)
+    h = normalised_hash_of_refused(pkg, p)
+    p.write_text("\n".join(("\\* a comment line\n" + ln + "   \r") if i == 20 else ln + "\r" for i, ln in enumerate(text.split("\n")))
+                 + "\n(* block\n (* nested *) comment *)\n\n")
+    assert normalised_hash_of_refused(pkg, p) == h
+    p.write_text(text.replace("AcknowledgedWriteNotLost == TRUE", "AcknowledgedWriteNotLost == TRUE \\/ FALSE"))
+    assert normalised_hash_of_refused(pkg, p) != h
+    # explicit override: loads, loudly, and is NOT reported as verified; the file's own hash and action locations are reported
     monkeypatch.setenv("VSR_B200_ALLOW_EDITED_SPEC", "1")
-    assert pkg.ModelChecker.from_cfg(REF_CFG, str(p)).info.spec_verified == 0
+    p.write_text(text)
+    mc = pkg.ModelChecker.from_cfg(REF_CFG, str(p))
+    assert mc.info.spec_verified == 0
+    fnv = 0xcbf29ce484222325
+    for c in text.encode():
+        fnv = ((fnv ^ c) * 0x100000001b3) & 0xFFFFFFFFFFFFFFFF
+    assert mc.info.spec_hash == fnv
+    lines = text.split("\n")
+    for a, name in enumerate(pkg.ACTION_NAMES):
+        want = "Unknown location" if a == 0 else "line %d, col 5 to line %d, col 21 of module VSR" % (
+            lines.index(name + " ==") + 2, lines.index(name + " ==") + 3)
+        assert mc.action_location(a) == want, name
 
 
-@needs_reference
+@pytest.mark.parametrize("edit,frag", [
+    (lambda t: t.replace("MODULE VSR", "MODULE VR_STATE_TRANSFER"), "MODULE VSR"),
+    (lambda t: t.replace(", aux_client_acked", ""), "VARIABLES"),
+    (lambda t: t.replace("    \\/ SendGetState\n", "    \\/ SendStateTransfer\n"), "disjunct"),
+    (lambda t: t.replace("TestInv == TRUE\n", ""), "TestInv"),
+])
+def test_other_specs_are_refused_even_with_the_override(pkg, tmp_path, monkeypatch, edit, frag):
+    """another module (the analysis specs are `MODULE VR_...`) or another outline is refused outright: the override only
+    admits edited definition bodies"""
+    p = tmp_path / "VSR.tla"
+    p.write_text(edit(stand_in_spec(pkg)))
+    normalised_hash_of_refused(pkg, p)
+    monkeypatch.setenv("VSR_B200_ALLOW_EDITED_SPEC", "1")
+    with pytest.raises(pkg.VsrError) as e:
+        pkg.ModelChecker.from_cfg(REF_CFG, str(p))
+    assert e.value.rc == 150 and frag in str(e.value), str(e.value)
+
+
 def test_readme_constants_load(pkg, tmp_path):
     """README.md:13-18: the user edits only the constants"""
     cfg = open(REF_CFG).read().replace("Values = {v1, v2}", "Values = {v1, v2, v3}").replace("StartViewOnTimerLimit = 2", "StartViewOnTimerLimit = 3")
     p = tmp_path / "VSR.cfg"
     p.write_text(cfg)
-    mc = pkg.ModelChecker.from_cfg(str(p), REF_TLA)
+    mc = pkg.ModelChecker.from_cfg(str(p))
     assert (mc.info.value_count, mc.info.start_view_on_timer_limit, mc.info.state_bytes) == (3, 3, 64)
 
 
-@needs_reference
-def test_other_specs_are_refused(pkg):
-    other = "/root/reference/vsr-revisited/paper/analysis/03-state-transfer/VR_STATE_TRANSFER.tla"
-    with pytest.raises(pkg.VsrError) as e:
-        pkg.ModelChecker.from_cfg(REF_CFG, other)
-    assert e.value.rc == 150
-
-
-@needs_reference
 @pytest.mark.parametrize("rel", ["analysis/03-state-transfer/VR_STATE_TRANSFER.cfg", "analysis/01-view-changes/VR_INC_RESEND.cfg"])
 def test_analysis_cfgs_are_refused_loudly(pkg, rel):
-    """they use SPECIFICATION / PROPERTY (liveness) — out of scope, must not be silently accepted"""
+    """the upstream analysis/ cfgs use SPECIFICATION / PROPERTY (liveness) — out of scope, must not be silently accepted"""
     with pytest.raises(pkg.VsrError) as e:
-        pkg.ModelChecker.from_cfg("/root/reference/vsr-revisited/paper/" + rel)
+        pkg.ModelChecker.from_cfg(os.path.join(GOLDEN, os.path.basename(rel)))
     assert e.value.rc == 151
 
 

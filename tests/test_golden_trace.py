@@ -10,7 +10,7 @@ import zlib
 import pytest
 
 import orc
-from conftest import REF_TRACE, needs_reference
+from conftest import REF_TRACE
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 FIXTURE = os.path.join(HERE, "golden", "state_transfer_trace.json")
@@ -105,7 +105,6 @@ def test_product_printer_equals_oracle_printer(pkg):
         assert mc.flat_to_tla(s) == orc.print_flat(q, s, True)
 
 
-@needs_reference
 def test_oracle_printer_reproduces_reference_file_byte_for_byte(pkg):
     """parse -> print of the reference file gives the file back (17-variable form it was written in; location strings
     carried through): pins value syntax, variable order, record field order and the ordering of the message bag"""
@@ -116,7 +115,6 @@ def test_oracle_printer_reproduces_reference_file_byte_for_byte(pkg):
     assert buf.raw[:n] == text
 
 
-@needs_reference
 def test_fixture_is_current(pkg):
     """the committed fixture equals what the generating script makes from the reference file today"""
     fx, states = load_fixture(pkg)
@@ -130,13 +128,12 @@ def test_fixture_is_current(pkg):
         assert bytes(flats[i]) == bytes(states[i])
 
 
-@needs_reference
 def test_dump_trace_format_matches_reference_shape(pkg):
     """product `-dumpTrace tlc` text for the golden behaviour: same record skeleton as the reference file (the current
-    spec has three more variables and other line numbers, so compare structure, not bytes)"""
-    from conftest import REF_TLA
+    spec has three more variables and other line numbers, so compare structure, not bytes; the locations the product reads
+    from VSR.tla are checked in test_boundary.py::test_shipped_cfg_and_spec_load_unchanged)"""
     fx, states = load_fixture(pkg)
-    mc = pkg.ModelChecker.from_cfg_text(pkg.cfg_text(3, ["v1", "v2", "v3"], 3, symmetry=False), REF_TLA)
+    mc = pkg.ModelChecker.from_cfg_text(pkg.cfg_text(3, ["v1", "v2", "v3"], 3, symmetry=False))
     trace = [(EXPECTED_ACTIONS[i], mc.pack(states[i])) for i in range(24)]
     text = mc.dump_trace_tlc(trace)
     ref = open(REF_TRACE).read()
@@ -144,4 +141,3 @@ def test_dump_trace_format_matches_reference_shape(pkg):
     drop = ("aux_restart |->", "rep_rec_number |->", "rep_rec_recv |->")
     ours = "\n".join(l for l in strip(text).split("\n") if not l.startswith(drop))
     assert ours == strip(ref)
-    assert 'location |-> "line 367, col 5 to line 394, col 122 of module VSR"' in text  # ReceiveClientRequest in the current spec
