@@ -120,8 +120,8 @@ typedef struct VsrRunOpts {
     /* checkpoint / recover: TLC's `-checkpoint <minutes>` and `-recover <dir>` (the reference's .gitignore:1 ignores TLC's
        states/ metadir, i.e. its users run with checkpoints).  checkpoint_path: file written at the first level boundary after
        checkpoint_seconds since the last one (0 = after every level; written to <path>.tmp and renamed, so an interrupted write
-       leaves the previous checkpoint intact); recover_path: continue the BFS from that file instead of Init.  With several
-       ranks every rank uses <path>.rank<r>.  NULL = off. */
+       leaves the previous checkpoint intact); recover_path: continue the BFS from that file instead of Init.  One rank uses
+       <path> itself; with several ranks every rank uses <path>.rank<r>.  NULL = off. */
     const char* checkpoint_path;
     const char* recover_path;
     double checkpoint_seconds;
@@ -159,13 +159,14 @@ typedef struct VsrStats {
 
 typedef struct VsrEngine VsrEngine;
 
-/* One-call BFS on one GPU.  Fails loudly (153) when no CUDA device is usable — there is no CPU
- * fallback.  If trace_out != NULL and a violation/deadlock is found, writes the counterexample
- * (packed states, trace_cap capacity) with its action ids; stats.trace_len is its length. */
+/* One-call BFS on one GPU: a world-1 engine running vsr_bfs_sharded.  Fails loudly (153) when no CUDA device is usable —
+ * there is no CPU fallback; a run that fails (CUDA, checkpoint file) returns its status with *stats all zero but rc.
+ * If trace_out != NULL and a violation/deadlock is found, writes the counterexample (packed states, trace_cap capacity)
+ * with its action ids; stats.trace_len is its length. */
 int vsr_bfs(const VsrModel* m, const VsrRunOpts* opts, VsrStats* stats, void* trace_out, uint8_t* trace_actions,
             size_t trace_cap);
 
-/* Stepwise engine (what vsr_bfs and vsr_bfs_sharded are made of).
+/* Stepwise engine (what vsr_bfs_sharded, and through it vsr_bfs, is made of).
  * rank/world: this engine owns the fingerprints f with owner(f) == rank (world = 1, 2, 4 or 8: the high bits of f). */
 int vsr_engine_create(const VsrModel* m, const VsrRunOpts* opts, int rank, int world, VsrEngine** out, char* err,
                       size_t errcap);
@@ -176,8 +177,6 @@ int vsr_engine_record_bytes(const VsrEngine* e);
 int vsr_engine_seed_init(VsrEngine* e);                       /* inserts Init if this rank owns it */
 /* one launch of the wavefront kernel over the whole current frontier (world = 1: that is the level) */
 int vsr_engine_expand(VsrEngine* e);
-/* same for frontier states [first, first + count) only */
-int vsr_engine_expand_part(VsrEngine* e, uint64_t first, uint64_t count);
 /* world > 1, one step = one launch: expand frontier states [first, first + count) — successors owned here are inserted,
  * the others are stored into their owners' inboxes (half `parity` of the double buffer) by the kernel itself — then insert
  * the records the peers stored HERE in the previous step: drain_counts[s] from rank s (NULL = none).  sent_out[d] = records
@@ -212,13 +211,12 @@ int vsr_engine_lookup(VsrEngine* e, const void* state, int* level_out, int* owne
  * with the file: vsr_bfs / vsr_bfs_sharded store the job's running totals there.  150 = not a checkpoint of this model. */
 int vsr_engine_checkpoint(VsrEngine* e, const char* path, const VsrStats* totals);
 int vsr_engine_recover(VsrEngine* e, const char* path, VsrStats* totals_out);
-/* forget everything explored (clears the seen-set, keeps the allocations): ready for seed_init again */
+/* forget everything explored (clears the seen-set unless nothing was inserted since create or the last reset, keeps the
+ * allocations): ready for seed_init again */
 int vsr_engine_reset(VsrEngine* e);
 const char* vsr_engine_last_error(const VsrEngine* e);
 /* with opts.collect_levels: number of states first seen at depth `level` (1-based) and, if host_out has room, a copy */
 uint64_t vsr_engine_collected(const VsrEngine* e, int level, void* host_out, uint64_t cap_states);
-/* Rebuild the counterexample ending at local state id (single-rank engines). */
-int vsr_engine_build_trace(VsrEngine* e, uint64_t local_id, void* trace_out, uint8_t* trace_actions, size_t trace_cap);
 
 /* ---- several GPUs of one node (SURVEY §8e: TLC's `-workers` / distributed mode).  One rank per GPU — processes
  * (torchrun) or threads of one process — fingerprint space split by its high bits.  The ranks coordinate through a
@@ -249,10 +247,12 @@ int vsr_engine_attach_group(VsrEngine* e, VsrGroup* g, uint64_t inbox_records);
 int vsr_engine_attach_staged(VsrEngine* e, uint64_t inbox_records, void** stage_out, void** inbox_out, uint64_t* cap_out);
 int vsr_engine_detach(VsrEngine* e);                                 /* collective when attached to a group */
 uint64_t vsr_engine_default_inbox_records(const VsrEngine* e);
-/* The whole BFS, called by every rank of the group with the same opts; all ranks return the same rc and the same totals
- * (records_sent / received, bytes_* and kernel_launches are this rank's).  part_states = frontier states per rank and step
- * (0 = from the inbox size).  On a violation / deadlock trace_cands[0 .. *trace_len) is the candidate chain from Init,
- * walked across ranks: vsr_replay_candidates turns it into the literal behaviour. */
+/* The whole BFS, called by every rank of the group with the same opts — or on a world-1 engine, which needs no group; all
+ * ranks return the same rc and the same totals (records_sent / received, bytes_* and kernel_launches are this rank's).
+ * part_states = frontier states per rank and step (0 = from the inbox size; one rank expands its whole frontier in one
+ * step).  On a violation / deadlock trace_cands[0 .. *trace_len) is the candidate chain from Init, walked across ranks:
+ * vsr_replay_candidates turns it into the literal behaviour.  *stats is written when the search reaches a verdict; a run
+ * that fails (CUDA, the group, a checkpoint file) returns its status and leaves *stats untouched. */
 int vsr_bfs_sharded(VsrEngine* e, const VsrRunOpts* opts, uint64_t part_states, VsrStats* stats, uint32_t* trace_cands, int* trace_len,
                     size_t trace_cap);
 /* `vsrmc -gpus N`: the same from ONE process, one thread per GPU (devices opts->device ... + ngpus - 1) */

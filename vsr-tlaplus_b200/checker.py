@@ -143,9 +143,9 @@ EXPORTED_SYMBOLS = [
     "vsr_load", "vsr_load_cfg_text", "vsr_model_create", "vsr_model_free", "vsr_model_info", "vsr_init", "vsr_successors", "vsr_enabled_candidates",
     "vsr_canon", "vsr_fingerprint", "vsr_fingerprint_bytewise", "vsr_aux_key", "vsr_owner_rank", "vsr_invariant", "vsr_unpack", "vsr_pack", "vsr_state_to_tla",
     "vsr_flat_to_tla", "vsr_action_name", "vsr_action_location", "vsr_bfs", "vsr_engine_create", "vsr_engine_destroy",
-    "vsr_engine_record_bytes", "vsr_engine_seed_init", "vsr_engine_expand", "vsr_engine_expand_part", "vsr_engine_step",
+    "vsr_engine_record_bytes", "vsr_engine_seed_init", "vsr_engine_expand", "vsr_engine_step",
     "vsr_engine_insert_records", "vsr_engine_finish_level", "vsr_engine_frontier_size", "vsr_engine_read_frontier",
-    "vsr_engine_trace_record", "vsr_engine_stats", "vsr_engine_reset", "vsr_engine_checkpoint", "vsr_engine_recover", "vsr_engine_lookup", "vsr_engine_last_error", "vsr_engine_collected", "vsr_engine_build_trace",
+    "vsr_engine_trace_record", "vsr_engine_stats", "vsr_engine_reset", "vsr_engine_checkpoint", "vsr_engine_recover", "vsr_engine_lookup", "vsr_engine_last_error", "vsr_engine_collected",
     "vsr_replay_candidates", "vsr_probe_bench", "vsr_simulate", "vsr_walk", "vsr_version",
     "vsr_group_open", "vsr_group_open_local", "vsr_group_close", "vsr_group_barrier", "vsr_group_allgather", "vsr_group_abort",
     "vsr_group_set_timeout", "vsr_group_rank", "vsr_group_world", "vsr_group_last_error",
@@ -217,7 +217,6 @@ def load_library(path: Optional[str] = None) -> C.CDLL:
                                   C.c_size_t]
     lib.vsr_engine_seed_init.argtypes = [vp]
     lib.vsr_engine_expand.argtypes = [vp]
-    lib.vsr_engine_expand_part.argtypes = [vp, u64, u64]
     lib.vsr_engine_insert_records.argtypes = [vp, vp, u64]
     lib.vsr_engine_finish_level.argtypes = [vp, C.POINTER(VsrLevelInfo)]
     lib.vsr_engine_frontier_size.argtypes = [vp]
@@ -233,7 +232,6 @@ def load_library(path: Optional[str] = None) -> C.CDLL:
     lib.vsr_engine_last_error.restype = cp
     lib.vsr_engine_collected.argtypes = [vp, C.c_int, vp, u64]
     lib.vsr_engine_collected.restype = u64
-    lib.vsr_engine_build_trace.argtypes = [vp, u64, vp, C.POINTER(C.c_uint8), C.c_size_t]
     lib.vsr_replay_candidates.argtypes = [vp, C.POINTER(C.c_uint32), C.c_int, vp, C.POINTER(C.c_uint8), C.c_size_t]
     lib.vsr_simulate.argtypes = [vp, C.POINTER(VsrSimOpts), C.POINTER(VsrSimStats), vp, C.POINTER(C.c_uint8), C.c_size_t]
     lib.vsr_walk.argtypes = [vp, u64, u64, C.c_int, C.POINTER(C.c_uint32), C.POINTER(C.c_int)]
@@ -487,11 +485,11 @@ class ModelChecker:
             trace=trace or [], levels=levels or [])
 
     def check(self, **kw) -> CheckResult:
-        """One-GPU BFS through the single C-ABI call ``vsr_bfs`` (counterexample included)."""
-        collect = kw.get("collect_levels", False)
-        if collect:
-            return self._check_stepwise(**kw)
+        """One-GPU BFS through the single C-ABI call ``vsr_bfs`` (counterexample included).  With collect_levels=True the
+        same loop, ``vsr_bfs_sharded`` on a one-rank engine, runs on an engine kept open to read every level's states back."""
         o = self.run_opts(**kw)
+        if o.collect_levels:
+            return self._check_collecting_levels(o)
         st = VsrStats()
         cap = 512
         tr = self._buf(cap)
@@ -499,20 +497,41 @@ class ModelChecker:
         rc = self._lib.vsr_bfs(self._h, C.byref(o), C.byref(st), tr, acts, cap)
         if rc == 153:
             raise VsrError(rc, "no usable CUDA device / CUDA failure (the BFS has no CPU fallback), or a checkpoint file could not be read / written")
-        raw = bytes(tr)
-        sb = self.state_bytes
-        trace = [(ACTION_NAMES[acts[i]], raw[i * sb:(i + 1) * sb]) for i in range(int(st.trace_len))]
-        return self.result_from_stats(st, rc, trace)
+        return self.result_from_stats(st, rc, self._trace(tr, acts, int(st.trace_len)))
 
-    def _trace_from_cands(self, cands, n: int) -> List[Tuple[str, bytes]]:
-        cap = n + 1
-        out = self._buf(cap)
-        acts = (C.c_uint8 * cap)()
-        m = self._lib.vsr_replay_candidates(self._h, cands, n, out, acts, cap)
-        if m < 0:
-            raise VsrError(255, "trace replay failed")
-        raw, sb = bytes(out), self.state_bytes
-        return [(ACTION_NAMES[acts[i]], raw[i * sb:(i + 1) * sb]) for i in range(m)]
+    def _check_collecting_levels(self, o: VsrRunOpts) -> CheckResult:
+        lib = self._lib
+        e = C.c_void_p()
+        err = C.create_string_buffer(512)
+        rc = lib.vsr_engine_create(self._h, C.byref(o), 0, 1, C.byref(e), err, len(err))
+        if rc:
+            raise VsrError(rc, err.value.decode())
+        try:
+            st = VsrStats()
+            cap = 4096
+            cands = (C.c_uint32 * cap)()
+            n = C.c_int(0)
+            rc = lib.vsr_bfs_sharded(e, C.byref(o), 0, C.byref(st), cands, C.byref(n), cap)
+            if rc not in (0, 11, 12, 152, 255):
+                raise VsrError(rc, lib.vsr_engine_last_error(e).decode())
+            levels = []
+            sb = self.state_bytes
+            for lv in range(1, int(st.num_levels) + 1):
+                k = lib.vsr_engine_collected(e, lv, None, 0)
+                buf = (C.c_uint8 * (k * sb))()
+                lib.vsr_engine_collected(e, lv, buf, k)
+                levels.append(bytes(buf))
+        finally:
+            lib.vsr_engine_destroy(e)
+        trace = replay_trace(self, cands[:n.value]) if st.trace_len else []
+        if trace:  # as vsr_bfs reports it: the INVARIANT bits the counterexample's last state violates
+            st.violation_mask = self.invariant(trace[-1][1])
+        return self.result_from_stats(st, rc, trace, levels)
+
+    def _trace(self, buf, acts, n: int) -> List[Tuple[str, bytes]]:
+        """the first n (action name, packed state) pairs of a trace buffer the library filled"""
+        raw, sb = bytes(buf), self.state_bytes
+        return [(ACTION_NAMES[acts[i]], raw[i * sb:(i + 1) * sb]) for i in range(n)]
 
     def check_multi(self, gpus: int, inbox_records: int = 0, part_states: int = 0, **kw) -> CheckResult:
         """The BFS sharded over `gpus` GPUs from THIS process (one thread per GPU): ``vsr_bfs_multi``, what `vsrmc -gpus N` runs."""
@@ -525,9 +544,7 @@ class ModelChecker:
         rc = self._lib.vsr_bfs_multi(self._h, C.byref(o), gpus, inbox_records, part_states, C.byref(st), tr, acts, cap, err, len(err))
         if rc in (151, 153):
             raise VsrError(rc, err.value.decode() or "no usable CUDA devices: the BFS has no CPU fallback")
-        raw, sb = bytes(tr), self.state_bytes
-        trace = [(ACTION_NAMES[acts[i]], raw[i * sb:(i + 1) * sb]) for i in range(int(st.trace_len))]
-        return self.result_from_stats(st, rc, trace)
+        return self.result_from_stats(st, rc, self._trace(tr, acts, int(st.trace_len)))
 
     def simulate(self, num_walks: int = 1 << 20, depth: int = 100, seed: int = 1, device: int = 0, probe_walks: int = 0):
         """TLC's `-simulate -depth N`: random behaviours on the GPU.  Returns (VsrSimStats, trace) — the trace is the
@@ -555,66 +572,14 @@ class ModelChecker:
         n = self._lib.vsr_walk(self._h, seed, walk, depth, cands, C.byref(va))
         return [int(cands[i]) for i in range(n)], int(va.value)
 
-    def _check_stepwise(self, **kw) -> CheckResult:
-        """Same BFS pumped level by level through the engine entry points (keeps every level for tests)."""
-        import time
-        o = self.run_opts(**kw)
-        lib = self._lib
-        e = C.c_void_p()
-        err = C.create_string_buffer(512)
-        rc = lib.vsr_engine_create(self._h, C.byref(o), 0, 1, C.byref(e), err, len(err))
-        if rc:
-            raise VsrError(rc, err.value.decode())
-        t0 = time.time()
-        try:
-            li = VsrLevelInfo()
-            result, complete, bad = 0, False, None
-            rc = lib.vsr_engine_seed_init(e) or lib.vsr_engine_finish_level(e, C.byref(li))
-            level = 1
-            while not rc:
-                if li.error_code:
-                    result = 255
-                    break
-                if li.overflow:
-                    result = 152
-                    break
-                if li.violation:
-                    result, bad = 12, int(li.violation_id)
-                    if o.stop_on_violation:
-                        break
-                if li.deadlock:
-                    result, bad = 11, int(li.deadlock_id)
-                    break
-                if lib.vsr_engine_frontier_size(e) == 0:
-                    complete = True
-                    break
-                if o.max_depth and level >= o.max_depth:
-                    break
-                rc = lib.vsr_engine_expand(e) or lib.vsr_engine_finish_level(e, C.byref(li))
-                level += 1
-            if rc:
-                raise VsrError(rc, lib.vsr_engine_last_error(e).decode())
-            st = VsrStats()
-            lib.vsr_engine_stats(e, C.byref(st))
-            st.depth = st.num_levels
-            st.complete = int(complete)
-            st.queue = 0 if complete else lib.vsr_engine_frontier_size(e)
-            st.seconds_total = time.time() - t0
-            levels = []
-            sb = self.state_bytes
-            for lv in range(1, int(st.num_levels) + 1):
-                n = lib.vsr_engine_collected(e, lv, None, 0)
-                buf = (C.c_uint8 * (n * sb))()
-                lib.vsr_engine_collected(e, lv, buf, n)
-                levels.append(bytes(buf))
-            trace = []
-            if bad is not None and o.keep_trace:
-                cap = 512
-                tr = self._buf(cap)
-                acts = (C.c_uint8 * cap)()
-                n = lib.vsr_engine_build_trace(e, bad, tr, acts, cap)
-                raw = bytes(tr)
-                trace = [(ACTION_NAMES[acts[i]], raw[i * sb:(i + 1) * sb]) for i in range(max(n, 0))]
-            return self.result_from_stats(st, result, trace, levels)
-        finally:
-            lib.vsr_engine_destroy(e)
+
+def replay_trace(mc: ModelChecker, cands: Sequence[int]) -> List[Tuple[str, bytes]]:
+    """Literal behaviour (fixed value names) from the candidate chain of a counterexample."""
+    n = len(cands)
+    cap = n + 1
+    out = mc._buf(cap)
+    acts = (C.c_uint8 * cap)()
+    m = mc._lib.vsr_replay_candidates(mc._h, (C.c_uint32 * max(n, 1))(*cands), n, out, acts, cap)
+    if m < 0:
+        raise VsrError(255, "trace replay failed")
+    return mc._trace(out, acts, m)

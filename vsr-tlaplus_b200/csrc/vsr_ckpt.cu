@@ -241,6 +241,7 @@ int vsr_engine_recover(VsrEngine* e, const char* path, VsrStats* totals_out) {
     }
     int rc = vsr_engine_reset(e);
     if (rc) return rc;
+    e->table_clean = false;
     CK(cudaStreamSynchronize(e->stream));
     std::vector<uint8_t> host;
     /* 1. the frontier, into buffer 0 */

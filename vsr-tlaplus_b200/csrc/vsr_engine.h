@@ -1,7 +1,7 @@
 /*
- * vsr_engine.h — internal: the engine object behind the opaque VsrEngine of include/vsr_b200.h, shared by vsr_gpu.cu (one
- * GPU: create / seed / expand / finish_level, vsr_bfs) and vsr_shard.cu (several GPUs: inboxes, the step that expands and
- * drains, vsr_bfs_sharded / vsr_bfs_multi).
+ * vsr_engine.h — internal: the engine object behind the opaque VsrEngine of include/vsr_b200.h, shared by vsr_gpu.cu (the
+ * engine's steps: create / seed / step / finish_level / reset), vsr_shard.cu (the exchange between ranks and the level loop
+ * vsr_bfs_sharded with its wrappers vsr_bfs / vsr_bfs_multi) and vsr_ckpt.cu (checkpoint / recover).
  */
 #ifndef VSR_ENGINE_H
 #define VSR_ENGINE_H
@@ -68,6 +68,7 @@ struct VsrEngine {
     uint64_t next_base = 0;      /* local id the next level starts at */
     int level = 0;               /* depth of the current frontier (Init = 1) */
     bool level_open = false;     /* counters reset for the level being generated */
+    bool table_clean = false;    /* the seen-set is all zero (since create or reset, nothing inserted): reset skips the memset */
     VsrStats st;
     double level_ms_acc = 0;
     double level_ms_insert_acc = 0; /* the part of level_ms_acc spent in launches that only insert records from peers */

@@ -1,8 +1,7 @@
 /*
- * vsr_gpu.cu — host driver of the BFS wavefront and the GPU half of the C ABI
- * (vsr_bfs, vsr_engine_*; include/vsr_b200.h).  "Thin C++ driver that pumps wavefronts":
- * per level one expand launch (plus insert launches for records received from peer ranks),
- * one small counter read-back, swap frontiers.  Kernels: vsr_gpu.cuh.
+ * vsr_gpu.cu — the engine's steps behind the C ABI (vsr_engine_*; include/vsr_b200.h), vsr_simulate and vsr_probe_bench.
+ * Per level one expand launch on each step (which also inserts the records peer ranks pushed here), one small counter
+ * read-back, swap frontiers.  The level loop that drives these steps is vsr_bfs_sharded (vsr_shard.cu).  Kernels: vsr_gpu.cuh.
  * There is NO CPU fallback: without a usable CUDA device every entry point returns 153.
  */
 #include <stddef.h>
@@ -158,6 +157,7 @@ int vsr_engine_create(const VsrModel* m, const VsrRunOpts* opts, int rank, int w
     e->st.bytes_frontier = 2 * fcap * S;
     e->st.bytes_h2d += 8 * 256 * 8;
     if ((ce = cudaStreamSynchronize(e->stream)) != cudaSuccess) return bail("sync", ce);
+    e->table_clean = true;
     *out = e;
     return 0;
 }
@@ -199,6 +199,7 @@ int vsr_engine_seed_init(VsrEngine* e) {
     int rc = engine_reset_level(e);
     if (rc) return rc;
     if (owner != e->rank) return 0;
+    e->table_clean = false;
     RecHdr* h = (RecHdr*)(rec.data() + e->g->bytes);
     h->fp = fp;
     h->tm = make_trec(ROOT_GID, 0) | (1ull << 56); /* no parent; stands for one generated state */
@@ -257,6 +258,7 @@ int vsr_engine_step(VsrEngine* e, uint64_t first, uint64_t count, int parity, co
     }
     if (sent_out) memset(sent_out, 0, sizeof(uint32_t) * e->world);
     if (count == 0 && drain_total == 0) return 0;
+    e->table_clean = false;
     CK(cudaMemsetAsync(&e->ctr->work_next, 0, sizeof(DevCounters) - offsetof(DevCounters, work_next), e->stream)); /* work_next, drain_next, send_count[] */
     const uint64_t spb = (uint64_t)e->g->states_per_block;
     uint64_t want_blocks = (count + spb - 1) / spb;
@@ -284,8 +286,6 @@ int vsr_engine_step(VsrEngine* e, uint64_t first, uint64_t count, int parity, co
     return 0;
 }
 
-int vsr_engine_expand_part(VsrEngine* e, uint64_t first, uint64_t count) { return vsr_engine_step(e, first, count, 0, nullptr, nullptr); }
-
 int vsr_engine_expand(VsrEngine* e) { return vsr_engine_step(e, 0, e->n_cur, 0, nullptr, nullptr); }
 
 int vsr_engine_insert_records(VsrEngine* e, const void* dev_records, uint64_t n) {
@@ -294,6 +294,7 @@ int vsr_engine_insert_records(VsrEngine* e, const void* dev_records, uint64_t n)
         if (rc) return rc;
     }
     if (n == 0) return 0;
+    e->table_clean = false;
     InsertParams q;
     fill_params(e, q.e);
     q.recs = (const uint8_t*)dev_records;
@@ -462,7 +463,8 @@ int vsr_engine_lookup(VsrEngine* e, const void* state, int* level_out, int* owne
 }
 
 int vsr_engine_reset(VsrEngine* e) {
-    CK(cudaMemsetAsync(e->table, 0, e->table_cap * 16, e->stream));
+    if (!e->table_clean) CK(cudaMemsetAsync(e->table, 0, e->table_cap * 16, e->stream)); /* tens of GB: once per run, not twice */
+    e->table_clean = true;
     const uint64_t tc = e->st.table_capacity, fc = e->st.frontier_capacity, bt = e->st.bytes_table, bf = e->st.bytes_frontier;
     memset(&e->st, 0, sizeof e->st);
     e->st.table_capacity = tc; e->st.frontier_capacity = fc; e->st.bytes_table = bt; e->st.bytes_frontier = bf;
@@ -486,95 +488,6 @@ uint64_t vsr_engine_collected(const VsrEngine* e, int level, void* host_out, uin
     const uint64_t n = v.size() / e->g->bytes;
     if (host_out && cap_states >= n) memcpy(host_out, v.data(), v.size());
     return n;
-}
-
-int vsr_engine_build_trace(VsrEngine* e, uint64_t local_id, void* trace_out, uint8_t* trace_actions, size_t trace_cap) {
-    if (e->world != 1) return -VSR_RC_ERROR; /* multi-rank chains are walked by the host that owns the collectives */
-    std::vector<uint32_t> cands;
-    uint64_t id = local_id;
-    const uint64_t root_parent = ROOT_GID;
-    for (int guard = 0; guard < 100000; guard++) {
-        uint64_t parent;
-        uint32_t cand;
-        if (vsr_engine_trace_record(e, id, &parent, &cand)) return -VSR_RC_ERROR;
-        if (parent == root_parent) break; /* Init */
-        cands.push_back(cand);
-        id = parent & ((1ull << 40) - 1);
-    }
-    std::vector<uint32_t> fwd(cands.rbegin(), cands.rend());
-    return vsr_replay_candidates(e->m, fwd.data(), (int)fwd.size(), trace_out, trace_actions, trace_cap);
-}
-
-int vsr_bfs(const VsrModel* m, const VsrRunOpts* opts, VsrStats* stats, void* trace_out, uint8_t* trace_actions, size_t trace_cap) {
-    if (!m || !opts || !stats) return VSR_RC_ERROR;
-    const double t0 = now_s();
-    VsrEngine* e = nullptr;
-    char err[256];
-    int rc = vsr_engine_create(m, opts, 0, 1, &e, err, sizeof err);
-    if (rc) {
-        memset(stats, 0, sizeof *stats);
-        stats->rc = rc;
-        if (opts->verbose) fprintf(stderr, "vsr_bfs: %s\n", err);
-        return rc;
-    }
-    const double t_setup = now_s() - t0;
-    VsrLevelInfo li;
-    memset(&li, 0, sizeof li);
-    int result = 0;
-    bool complete = false, bounded = false;
-    uint64_t bad_id = ~0ull;
-    if (opts->recover_path) { /* TLC -recover: continue from a checkpoint instead of Init */
-        rc = vsr_engine_recover(e, opts->recover_path, nullptr);
-        if (!rc && e->st.violation_level) { result = VSR_RC_VIOLATION; bad_id = e->st.violation_id; } /* found before the checkpoint, run continued past it */
-    } else {
-        rc = vsr_engine_seed_init(e);
-        if (!rc) rc = vsr_engine_finish_level(e, &li);
-    }
-    double last_ckpt = now_s();
-    while (!rc) {
-        if (li.error_code) { result = VSR_RC_ERROR; break; }
-        if (li.overflow) { result = VSR_RC_TOO_LARGE; break; }
-        if (li.violation && opts->stop_on_violation) { result = VSR_RC_VIOLATION; bad_id = li.violation_id; break; }
-        if (li.violation && !result) { result = VSR_RC_VIOLATION; bad_id = li.violation_id; }
-        if (li.deadlock) { result = VSR_RC_DEADLOCK; bad_id = li.deadlock_id; break; }
-        if (e->n_cur == 0) { complete = true; break; }
-        if (opts->max_depth && e->level >= opts->max_depth) { bounded = true; break; }
-        if (opts->max_states && e->st.distinct >= opts->max_states) { bounded = true; break; }
-        if (opts->max_seconds > 0 && now_s() - t0 >= opts->max_seconds) { bounded = true; break; }
-        if (e->level >= 254) { result = VSR_RC_TOO_LARGE; break; } /* 8-bit level tag in the seen-set */
-        if (opts->checkpoint_path && now_s() - last_ckpt >= opts->checkpoint_seconds) { /* TLC -checkpoint: at a level boundary */
-            rc = vsr_engine_checkpoint(e, opts->checkpoint_path, nullptr);
-            if (rc) break;
-            last_ckpt = now_s();
-            if (opts->verbose) fprintf(stderr, "Checkpointing of run %s completed (depth %d, %llu distinct states).\n", opts->checkpoint_path, e->level, (unsigned long long)e->st.distinct);
-        }
-        rc = vsr_engine_expand(e);
-        if (rc) break;
-        rc = vsr_engine_finish_level(e, &li);
-        if (opts->verbose && !rc)
-            fprintf(stderr, "depth %3d: %12llu new  %12llu generated  %8.3f ms\n", e->level, (unsigned long long)li.new_states,
-                    (unsigned long long)li.generated, li.ms);
-    }
-    /* a run that stops on a bound (-depth, max_states, max_seconds) leaves a checkpoint to continue from */
-    if (!rc && bounded && opts->checkpoint_path) rc = vsr_engine_checkpoint(e, opts->checkpoint_path, nullptr);
-    if (rc) result = rc;
-    VsrStats s = e->st;
-    s.rc = result;
-    s.complete = complete ? 1 : 0;
-    s.depth = s.num_levels;
-    s.queue = complete ? 0 : e->n_cur;
-    if (bad_id != ~0ull && trace_out && e->trace) {
-        int n = vsr_engine_build_trace(e, bad_id, trace_out, trace_actions, trace_cap);
-        s.trace_len = n > 0 ? n : 0;
-        if (n > 0 && result == VSR_RC_VIOLATION)
-            s.violation_mask = m->ops->invariant(&m->run, (const uint32_t*)((const uint8_t*)trace_out + (size_t)(n - 1) * m->ops->bytes));
-    }
-    s.seconds_total = now_s() - t0;
-    s.seconds_setup = t_setup;
-    *stats = s;
-    if (rc && opts->verbose) fprintf(stderr, "vsr_bfs: %s\n", e->last_error);
-    vsr_engine_destroy(e);
-    return result;
 }
 
 /* TLC `-simulate`: random walks on the GPU; a violating walk is re-walked on the host (same generator, same step

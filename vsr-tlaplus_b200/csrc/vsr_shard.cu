@@ -13,7 +13,9 @@
  *   vsr_engine_attach_group   allocate the inbox, exchange IPC handles through the group, map the peers
  *   vsr_engine_attach_staged  the same kernel writing into a LOCAL staging buffer, for a host that moves the records with
  *                             a collective instead (dist.ShardedBfs over torch.distributed: NCCL all-to-all, or gloo in tests)
- *   vsr_bfs_sharded           the level loop, called by every rank; all ranks return the same totals
+ *   vsr_bfs_sharded           the level loop, called by every rank; all ranks return the same totals.  It is also the loop of
+ *                             one GPU: with world 1 there is no group, and one step expands the whole frontier
+ *   vsr_bfs                   one GPU: a world-1 engine, vsr_bfs_sharded, the counterexample replayed
  *   vsr_bfs_multi             one process, one thread per GPU (vsrmc -gpus N)
  */
 #include <stdlib.h>
@@ -183,9 +185,10 @@ int vsr_engine_attach_staged(VsrEngine* e, uint64_t inbox_records, void** stage_
     return 0;
 }
 
-/* The level loop on every rank of the group.  All ranks take every decision from the same all-gathered numbers, so they
-   leave the loop together and report the same totals.  trace_cands / trace_len: the candidate chain from Init to the
-   violating (or deadlocked) state, walked across ranks; replay it with vsr_replay_candidates. */
+/* The level loop on every rank of the group, or on a world-1 engine without one.  All ranks take every decision from the
+   same all-gathered numbers, so they leave the loop together and report the same totals.  trace_cands / trace_len: the
+   candidate chain from Init to the violating (or deadlocked) state, walked across ranks; replay it with
+   vsr_replay_candidates.  *stats is written only when the search reaches a verdict, not when it fails (CUDA, checkpoint). */
 int vsr_bfs_sharded(VsrEngine* e, const VsrRunOpts* opts, uint64_t part_states, VsrStats* stats, uint32_t* trace_cands, int* trace_len, size_t trace_cap) {
     if (!e || !opts || !stats) return VSR_RC_ERROR;
     if (trace_len) *trace_len = 0;
@@ -196,7 +199,7 @@ int vsr_bfs_sharded(VsrEngine* e, const VsrRunOpts* opts, uint64_t part_states, 
     /* a step of S states per rank fills each peer segment with about S * (successor records per state) / W records.  The
        fan-out is measured, not assumed (2.7 per state on the shipped VSR.cfg, 16 with five replicas): each level's steps are
        sized from the previous level's ratio with a factor of two to spare (an overflow is detected, never silent) */
-    const bool auto_part = part_states == 0;
+    const bool auto_part = part_states == 0 || W == 1; /* one rank: no inbox, one step expands the whole frontier */
     double fanout = 16.0, seg_ratio = 0;
     uint64_t prev_frontier_total = 0;
     VsrStats tot;
@@ -205,13 +208,15 @@ int vsr_bfs_sharded(VsrEngine* e, const VsrRunOpts* opts, uint64_t part_states, 
     bool complete = false, bounded = false;
     uint64_t bad_gid = ~0ull;
     double kernel_ms = 0, insert_ms = 0;
-    /* checkpoints: every rank writes / reads <path>.rank<r> at the same level boundary (rank 0's clock decides when) */
-    const std::string ckpt_path = opts->checkpoint_path ? std::string(opts->checkpoint_path) + ".rank" + std::to_string(me) : std::string();
+    /* checkpoints: every rank writes / reads <path>.rank<r> at the same level boundary (rank 0's clock decides when); one
+       rank uses <path> itself */
+    const std::string rank_suffix = W > 1 ? ".rank" + std::to_string(me) : std::string();
+    const std::string ckpt_path = opts->checkpoint_path ? opts->checkpoint_path + rank_suffix : std::string();
     double last_ckpt = now_s();
     bool resumed = false;
     int rc;
     if (opts->recover_path) {
-        rc = vsr_engine_recover(e, (std::string(opts->recover_path) + ".rank" + std::to_string(me)).c_str(), &tot);
+        rc = vsr_engine_recover(e, (opts->recover_path + rank_suffix).c_str(), &tot);
         if (!rc) {
             resumed = true;
             level = e->level - 1; /* the loop's first pass stands at the checkpoint's level boundary without finishing a level */
@@ -280,8 +285,11 @@ int vsr_bfs_sharded(VsrEngine* e, const VsrRunOpts* opts, uint64_t part_states, 
             tot.level_sizes[level - 1] = n_new;
             tot.num_levels = level;
         }
-        if (opts->verbose && me == 0 && level >= 2 && !boundary_only)
-            fprintf(stderr, "depth %3d: %12llu new  %12llu generated  %8.3f ms (slowest of %d GPUs)\n", level, (unsigned long long)n_new, (unsigned long long)n_gen, ms, W);
+        if (opts->verbose && me == 0 && level >= 2 && !boundary_only) {
+            fprintf(stderr, "depth %3d: %12llu new  %12llu generated  %8.3f ms", level, (unsigned long long)n_new, (unsigned long long)n_gen, ms);
+            if (W > 1) fprintf(stderr, " (slowest of %d GPUs)", W);
+            fprintf(stderr, "\n");
+        }
         if (err) { result = VSR_RC_ERROR; tot.error_code = err; break; }
         if (ovf) { result = VSR_RC_TOO_LARGE; break; }
         if (viol && !tot.violation_level) {
@@ -303,7 +311,8 @@ int vsr_bfs_sharded(VsrEngine* e, const VsrRunOpts* opts, uint64_t part_states, 
             step_rc = vsr_engine_checkpoint(e, ckpt_path.c_str(), &tot); /* a failure travels to everybody in the next all-gather */
             last_ckpt = now_s();
             if (opts->verbose && me == 0 && !step_rc)
-                fprintf(stderr, "Checkpointing of run %s.rank* completed (depth %d, %llu distinct states).\n", opts->checkpoint_path, level, (unsigned long long)tot.distinct);
+                fprintf(stderr, "Checkpointing of run %s%s completed (depth %d, %llu distinct states).\n", opts->checkpoint_path, W > 1 ? ".rank*" : "", level,
+                        (unsigned long long)tot.distinct);
         }
         /* ---- the next level, in steps: step k expands part k and pushes into inbox half k & 1, and drains what the
            peers pushed here in step k - 1; one more launch drains the last part's records */
@@ -435,6 +444,43 @@ int vsr_bfs_sharded(VsrEngine* e, const VsrRunOpts* opts, uint64_t part_states, 
     return result;
 }
 
+/* the literal counterexample of a finished search from the candidate chain vsr_bfs_sharded walked (it set stats->trace_len
+   when it walked one): its length and the INVARIANT bits its last state violates */
+static void replay_counterexample(const VsrModel* m, const uint32_t* cands, int n, VsrStats* stats, void* trace_out, uint8_t* trace_actions,
+                                  size_t trace_cap) {
+    const int len = trace_out && stats->trace_len > 0 ? vsr_replay_candidates(m, cands, n, trace_out, trace_actions, trace_cap) : 0;
+    stats->trace_len = len > 0 ? len : 0;
+    if (len > 0) stats->violation_mask = m->ops->invariant(&m->run, (const uint32_t*)((const uint8_t*)trace_out + (size_t)(len - 1) * m->ops->bytes));
+}
+
+int vsr_bfs(const VsrModel* m, const VsrRunOpts* opts, VsrStats* stats, void* trace_out, uint8_t* trace_actions, size_t trace_cap) {
+    if (!m || !opts || !stats) return VSR_RC_ERROR;
+    const double t0 = now_s();
+    memset(stats, 0, sizeof *stats);
+    VsrEngine* e = nullptr;
+    char err[256];
+    int rc = vsr_engine_create(m, opts, 0, 1, &e, err, sizeof err);
+    if (rc) {
+        stats->rc = rc;
+        if (opts->verbose) fprintf(stderr, "vsr_bfs: %s\n", err);
+        return rc;
+    }
+    const double t_setup = now_s() - t0;
+    std::vector<uint32_t> cands(4096);
+    int n = 0;
+    rc = vsr_bfs_sharded(e, opts, 0, stats, trace_out ? cands.data() : nullptr, &n, cands.size());
+    if (stats->rc != rc) { /* failed before a verdict: *stats is still all zero */
+        stats->rc = rc;
+        if (opts->verbose) fprintf(stderr, "vsr_bfs: %s\n", e->last_error);
+    } else {
+        replay_counterexample(m, cands.data(), n, stats, trace_out, trace_actions, trace_cap);
+        stats->seconds_setup = t_setup;
+        stats->seconds_total = now_s() - t0;
+    }
+    vsr_engine_destroy(e);
+    return rc;
+}
+
 /* vsrmc -gpus N: one process, one thread per GPU; devices opts->device .. opts->device + ngpus - 1 */
 int vsr_bfs_multi(const VsrModel* m, const VsrRunOpts* opts, int ngpus, uint64_t inbox_records, uint64_t part_states, VsrStats* stats, void* trace_out,
                   uint8_t* trace_actions, size_t trace_cap, char* err, size_t errcap) {
@@ -493,12 +539,7 @@ int vsr_bfs_multi(const VsrModel* m, const VsrRunOpts* opts, int ngpus, uint64_t
             if (!errors[r].empty()) { snprintf(err, errcap, "GPU %d: %s", opts->device + r, errors[r].c_str()); break; }
     }
     *stats = st[0];
-    if ((rc == VSR_RC_VIOLATION || rc == VSR_RC_DEADLOCK || (rc == 0 && st[0].violation_level)) && trace_out && lens[0] >= 0 && st[0].trace_len > 0) {
-        const int n = vsr_replay_candidates(m, cands[0].data(), lens[0], trace_out, trace_actions, trace_cap);
-        stats->trace_len = n > 0 ? n : 0;
-        if (n > 0 && stats->violation_level)
-            stats->violation_mask = m->ops->invariant(&m->run, (const uint32_t*)((const uint8_t*)trace_out + (size_t)(n - 1) * m->ops->bytes));
-    } else stats->trace_len = 0;
+    replay_counterexample(m, cands[0].data(), lens[0], stats, trace_out, trace_actions, trace_cap);
     stats->seconds_total = now_s() - t0;
     return rc;
 }

@@ -30,6 +30,7 @@ import torch
 import torch.distributed as dist
 
 from . import checker as ck
+from .checker import replay_trace  # noqa: F401  (part of this module's interface: check_sharded, bench.py and the tests use it)
 
 I64_MAX = (1 << 63) - 1
 GID_SHIFT = 40             # global state id = rank << 40 | local id (vsr_gpu.cuh make_gid)
@@ -169,7 +170,8 @@ class GpuEngine:
     def run(self, max_depth: int = 0, max_seconds: float = 0.0, max_states: int = 0, stop_on_violation: bool = True,
             want_trace: bool = True, part_states: int = 0, verbose: bool = False, checkpoint_path: Optional[str] = None,
             recover_path: Optional[str] = None, checkpoint_seconds: float = 0.0) -> ShardedResult:
-        """checkpoint_path / recover_path: every rank writes / reads ``<path>.rank<r>`` at level boundaries (TLC -checkpoint / -recover)"""
+        """checkpoint_path / recover_path: TLC -checkpoint / -recover at level boundaries; with several ranks every rank writes /
+        reads ``<path>.rank<r>``, one rank ``<path>`` itself"""
         o = self._opts
         o.max_depth, o.max_seconds, o.max_states = max_depth, max_seconds, max_states
         o.stop_on_violation, o.verbose = int(stop_on_violation), int(verbose)
@@ -476,18 +478,3 @@ class ShardedBfs:
             cands.append(cand)
             gid = parent
         return cands[::-1]
-
-
-def replay_trace(mc: "ck.ModelChecker", cands: List[int]) -> List[Tuple[str, bytes]]:
-    """Literal behaviour (fixed value names) from the candidate chain of a counterexample."""
-    n = len(cands)
-    arr = (C.c_uint32 * max(n, 1))(*cands)
-    cap = n + 1
-    out = (C.c_uint8 * (cap * mc.state_bytes))()
-    acts = (C.c_uint8 * cap)()
-    m = mc._lib.vsr_replay_candidates(mc._h, arr, n, out, acts, cap)
-    if m < 0:
-        raise ck.VsrError(255, "trace replay failed")
-    raw = bytes(out)
-    sb = mc.state_bytes
-    return [(ck.ACTION_NAMES[acts[i]], raw[i * sb:(i + 1) * sb]) for i in range(m)]
